@@ -5,13 +5,16 @@ SGD lr 1e-4, fp32 with TF32 tensor-core convolutions, synthetic MNIST-shaped dat
 
     python bench.py --gpus N --steps K --warmup W                 # this framework
     python bench.py --impl reference --gpus N --steps K --warmup W # unmodified reference stack
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's results to DIR/*.npy
 
 N > 1 is launched one rank per GPU by ``python -m torch.distributed.run --nproc-per-node N ...``
 (RANK / LOCAL_RANK / WORLD_SIZE / MASTER_* from the environment).  Rank 0 prints ONE JSON line.
 
 Timed regions (both arms): W >= 3 untimed warm-up steps, then exactly K steps between
 barrier + torch.cuda.synchronize() on both sides, CUDA events on the launching stream, MAX over
-ranks.  ``value`` is the device-timed step with inputs rotating through a device-resident pool that
+ranks.  Inputs are seeded, so the same arguments give the same inputs on every run; ``--dump-outputs`` saves what
+the last device-timed step returned (its loss) and left behind (parameters, BatchNorm buffers) for comparing two
+builds output for output.  ``value`` is the device-timed step with inputs rotating through a device-resident pool that
 is larger than L2 (164 MB > 126 MB).  ``e2e`` is the same step driven end to end through the framework's
 own input path — ``data.MNIST`` on synthetic idx files -> ``DistributedSampler`` -> ``DataLoader(pin_memory=True)``
 -> H2D of every batch -> whole-step graph -> D2H of every loss — i.e. the loop of ``cli.dist_train``
@@ -25,6 +28,7 @@ import json
 import os
 import statistics
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -50,7 +54,13 @@ def parse():
     p.add_argument("--conv-impl", default="auto", choices=["auto", "simt", "tcgen05"])
     p.add_argument("--skip-e2e", action="store_true")
     p.add_argument("--skip-verify", action="store_true", help="skip the pre-timing cross-check against torch autograd (+NCCL)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the device-timed steps, write rank 0's loss of the last step and the parameters and buffers it left "
+                        "to DIR/<name>.npy (float32; integer buffers as float64)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
 
 
 def env_rank():
@@ -77,8 +87,10 @@ def window_stats(marks):
 
 
 def ensure_synthetic_mnist(local_rank: int) -> str:
-    """Synthetic idx files where both arms' MNIST datasets look for them (./data/MNIST/raw); written once."""
-    data_root = os.path.join(os.getcwd(), "data")
+    """Synthetic idx files in ``<data_root>/MNIST/raw``, where both arms' MNIST datasets look for them; returns data_root.
+    They live in a per-user temporary directory, not in the working directory (which may be the read-only source
+    tree), and are written once and reused: their content is fixed by a seed."""
+    data_root = os.path.join(tempfile.gettempdir(), f"pdt_bench_{os.getuid()}", "data")
     marker = os.path.join(data_root, "MNIST", "raw", ".synthetic_ready")
     if local_rank == 0 and not os.path.exists(marker):
         sys.path.insert(0, os.path.join(ROOT, "baseline"))
@@ -92,6 +104,22 @@ def ensure_synthetic_mnist(local_rank: int) -> str:
             raise RuntimeError("timed out waiting for the synthetic MNIST files")
         time.sleep(0.05)
     return data_root
+
+
+def snapshot_outputs(loss, module) -> dict:
+    """Host copies of what a training step hands its caller: the loss it returned, and the parameters and buffers it left."""
+    out = {"loss": loss}
+    out.update({f"param.{k}": v for k, v in module.named_parameters()})
+    out.update({f"buffer.{k}": v for k, v in module.named_buffers()})
+    return {k: v.detach().cpu().clone() for k, v in out.items()}
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t.float() if t.is_floating_point() else t.double()).numpy())
 
 
 # =====================================================================================================
@@ -272,6 +300,8 @@ def run_ours(args):
     with ClockSampler(gpu_index=local_rank, period_ms=100) as clocks:
         ms_dev, _, eager_launches, windows = timed(dev_step, W, K)
         final_loss = float(last["loss"].detach())
+        # taken before the e2e run below trains the same model further (and replays overwrite the graph's loss tensor)
+        outputs = snapshot_outputs(last["loss"], ddp.module) if args.dump_outputs and rank == 0 else None
         # ---- end to end through the framework's own input path (the loop of cli.dist_train) -----------
         e2e = None
         if not args.skip_e2e:
@@ -378,6 +408,8 @@ def run_ours(args):
                                   "GraphedTrainStep(pinned images, pinned labels): H2D + whole-step graph replay; step.loss_to_host(): async D2H of every "
                                   "loss; blocking read of every 10th loss on rank 0, issued after the following step has been queued (the loop of "
                                   "cli.dist_train; cadence of ref ddp_example.py:93-95)"}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     pdt.destroy_process_group()
     if verify is not None and not verify["ok"]:
         if out is not None:
@@ -392,10 +424,8 @@ def run_ours(args):
 def _ensure_reference():
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     sys.path.insert(0, os.path.join(ROOT, "baseline"))
-    if not os.path.exists(os.path.join(ref_dir, "ddp_example.py")):
-        import install_ref
-
-        install_ref.install()
+    if not os.path.exists(os.path.join(ref_dir, "ddp_example.py")):   # installed by build(); the benchmark does not write the tree
+        raise FileNotFoundError(f"{ref_dir} has no ddp_example.py; build() installs the reference there")
     return ref_dir
 
 
@@ -472,6 +502,7 @@ def run_reference(args):
         ms_dev = float(t.item())
         windows = window_stats(marks)
         final_loss = float(loss.detach())
+        outputs = snapshot_outputs(loss, model.module) if args.dump_outputs and rank == 0 else None
         del model, optimizer
         dist.destroy_process_group()
 
@@ -483,12 +514,14 @@ def run_reference(args):
         e2e_err = None
         if not args.skip_e2e:
             try:
-                ensure_synthetic_mnist(local_rank)
-                e2e_ms = _reference_e2e(ref, args, rank, local_rank, world, W, K, base_port + 12)
+                data_root = ensure_synthetic_mnist(local_rank)
+                e2e_ms = _reference_e2e(ref, args, rank, local_rank, world, W, K, base_port + 12, data_root)
             except Exception as e:  # noqa: BLE001
                 e2e_err = f"{type(e).__name__}: {e}"[:300]
     if rank != 0:
         return None
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     imgs = BATCH * world * K
     out = {
         "metric": METRIC, "value": imgs / (ms_dev / 1e3), "unit": "images/s", "n_gpus": world, "steps": K, "warmup": W,
@@ -510,7 +543,7 @@ def run_reference(args):
     return out
 
 
-def _reference_e2e(ref, args, rank, local_rank, world, W, K, port):
+def _reference_e2e(ref, args, rank, local_rank, world, W, K, port, data_root):
     import io
     from contextlib import redirect_stdout
     from types import SimpleNamespace
@@ -548,11 +581,14 @@ def _reference_e2e(ref, args, rank, local_rank, world, W, K, port):
     ns = SimpleNamespace(gpus=world, epochs=epochs, backend="nccl", syncbn=args.syncbn, world_size=world,
                          init_method=f"tcp://127.0.0.1:{port}")
     tud.DataLoader = TimedLoader
+    cwd = os.getcwd()
+    os.chdir(os.path.dirname(data_root))   # the reference reads MNIST from ./data
     try:
         buf = io.StringIO()
         with redirect_stdout(buf):   # the reference prints every 10 steps; keep our stdout to one JSON line
             ref.dist_train(local_rank, ns)
     finally:
+        os.chdir(cwd)
         tud.DataLoader = Base
     if state["ms"] is None:
         raise RuntimeError(f"reference loop ended after {state['n']} steps, before warmup+steps={W + K}")

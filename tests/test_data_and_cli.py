@@ -15,10 +15,12 @@ from pytorch_distributed_train_b200.data import (MNIST, DataLoader, DistributedS
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_idx_roundtrip_and_mnist(tmp_path):
+def test_idx_roundtrip_and_mnist(tmp_path, monkeypatch):
     t = (torch.arange(2 * 28 * 28) % 251).to(torch.uint8).view(2, 28, 28)
     write_idx(str(tmp_path / "x-idx3-ubyte"), t)
     assert torch.equal(read_idx(str(tmp_path / "x-idx3-ubyte")), t)
+    # an offline machine, whatever this one is: the test must never open a connection to the dataset mirrors
+    monkeypatch.setattr(pdt.data.mnist, "network_reachable", lambda *a, **k: False)
     with pytest.raises(RuntimeError, match="no network is reachable"):
         MNIST(str(tmp_path / "none"), download=True)
     synthesize_mnist_files(str(tmp_path), n=300)
